@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's configuration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--blocks B] [--cls E50]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--blocks B] [--cls E50] [--dump-outputs DIR]
 
 metric  : "GB/s encode+decode on batched 64KiB blocks" -- raw (uncompressed) bytes per second through one encode pass
           plus one decode pass over the batch (the reference's convention: throughput numerator = uncompressed bytes in
@@ -61,7 +61,12 @@ def parse():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--sweep-blocks", type=int, default=1 << 17)
     p.add_argument("--hc-blocks", type=int, default=1 << 17)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last timed step returned as DIR/<name>.npy (rank 0's blocks), to compare two builds")
+    args = p.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs dumps the GPU path's outputs; --impl reference has none")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -281,6 +286,30 @@ class Workload:
         ev[0][0].record(); self.encode(); ev[0][1].record()
         for w in range(self.n_waves):
             ev[1 + w][0].record(); self.decode_wave(w); ev[1 + w][1].record()
+
+
+DUMP_SAMPLE_BLOCKS = 64
+
+
+def dump_outputs(work, out_dir):
+    """Writes what the last step returned to its caller as float32 arrays (byte values and lengths are exact in float32):
+    every block's compressed length and the bytes the decoder consumed, and, for a fixed seeded sample of the blocks whose
+    decoded bytes are still in the reused decode buffer (the last wave), their compressed bytes (zero past the length)
+    and decoded bytes.  40 MiB at the default 2^20 blocks."""
+    import numpy as np
+    torch = work.torch
+    torch.cuda.synchronize()
+    first = (work.n_waves - 1) * work.wave
+    blocks = np.sort(np.random.default_rng(0).choice(np.arange(first, work.n), min(DUMP_SAMPLE_BLOCKS, work.n - first), replace=False))
+    idx = torch.from_numpy(blocks).to(work.clen.device)
+    comp = work.slots.view(work.n, work.slot)[idx]
+    comp[torch.arange(work.slot, device=idx.device)[None, :] >= work.clen[idx].unsqueeze(1)] = 0
+    arrays = {"compressed_lengths": work.clen, "decode_consumed": work.used, "sample_blocks": blocks,
+              "compressed_sample": comp, "decoded_sample": work.out.view(work.wave, BLOCK)[idx - first]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a if isinstance(a, np.ndarray) else a.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if name == "sample_blocks" else np.float32))
 
 
 def measure_pair(work, steps, warmup, hc=False):
@@ -603,6 +632,8 @@ def main():
     roof_enc = {"kernel": "lz4_encode_fast_kernel", "bound": "hbm", "achieved": round(alg / t_enc / GB, 1), "peak": peak_hbm, "unit": "GB/s",
                 "frac": round(alg / t_enc / GB / peak_hbm, 4), "traffic": traffic_enc, "traffic_source": tsrc, "peak_source": peak_src,
                 "algorithmic_bytes_per_launch": int(alg), "launch_ms": round(t_enc * 1e3, 3)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(work, args.dump_outputs)
     del work
     torch.cuda.empty_cache()
 

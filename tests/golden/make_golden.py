@@ -5,6 +5,8 @@
 
 The reference ships no golden vectors of its own (SURVEY.md 8c); these are outputs of the reference itself on
 reproducible inputs (tests/cases.py), including the reference-defined AutoTest text (src/LZ4/LZ4Codec.cs:175-184).
+It also writes tests/golden/reference_results.json: the reference's return values and output digests for the inputs
+of tests/test_oracle.py's comparisons with the reference, computed by that module's own functions.
 """
 import hashlib
 import json
@@ -47,6 +49,34 @@ def main():
     json.dump({"source": "oracle/_ref (reference original/lz4.c + lz4hc.c, LZ4_ARCH64=1, LZ4_MK_OPT)", "cases": out},
               open(path, "w"), indent=1)
     print("wrote", path, len(out), "cases")
+    reference_results()
+
+
+def reference_results():
+    from lz4net_b200 import synth
+    from tests import test_oracle as t
+    rl = {m: [[n, t.encode_results(d, "ref")[0]] for n, d in t.random_length_inputs(m)] for m in cases.MODELS}
+    ar = [t.accept_reject_results(oracle.encode(d, impl="ref")[1], len(d), "ref") for _, d in t.accept_reject_inputs()]
+    comps, streams = t.corrupt_streams("ref")
+    cs = {"comp": t.digest(*comps), "verdicts": [t.unknown_result(c, n, "ref") for n, c in streams]}
+    # tests/test_kernels_emu.py: a block on which r93's LZ4HC gives up at the bound
+    d = synth.make_blocks("E0", 1, 65536, seed=3, first_block=1268)[0].tobytes()
+    cap = oracle.bound(len(d))
+    hc_bound = [oracle.encode_hc(d, cap=cap, impl="ref")[0], oracle.encode_hc(d, cap=cap + 4096, impl="ref")[0]]
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_results.json")
+    doc = {"source": "oracle/_ref (reference original/lz4.c + lz4hc.c, LZ4_ARCH64=1, LZ4_MK_OPT)",
+           "random_lengths": rl, "accept_reject": ar, "corrupt_streams": cs, "encode_hc_gives_up_at_the_bound": hc_bound}
+    with open(path, "w") as f:                  # one entry of each list or object per line: diffs stay readable
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {_one_entry_per_line(v)}" for k, v in doc.items()) + "\n}\n")
+    print("wrote", path)
+
+
+def _one_entry_per_line(v):
+    if isinstance(v, dict):
+        return "{\n" + ",\n".join(f" {json.dumps(k)}: {json.dumps(x)}" for k, x in v.items()) + "\n}"
+    if isinstance(v, list) and v and isinstance(v[0], (list, dict)):
+        return "[\n" + ",\n".join(" " + json.dumps(x) for x in v) + "\n]"
+    return json.dumps(v)
 
 
 if __name__ == "__main__":
