@@ -116,6 +116,19 @@ int64_t lz4b200_stream_encode(lz4b200_ctx* ctx, const void* src, int64_t n, int3
 int64_t lz4b200_stream_decoded_size(const void* src, int64_t n);     /* sum of rawLen over all chunks, <0 = malformed */
 int64_t lz4b200_stream_decode(lz4b200_ctx* ctx, const void* src, int64_t n, void* dst, int64_t dst_cap);
 
+/* LZ4Stream framing on device memory (src, dst on the context's GPU).  Ordered on `stream`: the call waits for
+ * work already queued there, and returns once its result is known.
+ * Each call returns exactly what its host twin above returns for the same bytes -- bytes written, the total raw size,
+ * LZ4B200_E_ARG (dst_cap below lz4b200_stream_bound / below the total; no byte of dst is written then) or
+ * LZ4B200_E_FORMAT -- and the encoder writes the same bytes.  src and dst may have any alignment; no byte outside
+ * [src, src + n) is parsed.  The compressed bytes never cross PCIe: only the sizes come back to the host.
+ * decoded_size walks the chunk headers on the device (one thread: each header's position depends on the one before);
+ * decode walks them again, then copies the stored chunks and decodes all compressed ones in one batch. */
+int64_t lz4b200_stream_encode_device(lz4b200_ctx* ctx, const void* src, int64_t n, int32_t block_size,
+                                     int high_compression, void* dst, int64_t dst_cap, void* stream);
+int64_t lz4b200_stream_decoded_size_device(lz4b200_ctx* ctx, const void* src, int64_t n, void* stream);
+int64_t lz4b200_stream_decode_device(lz4b200_ctx* ctx, const void* src, int64_t n, void* dst, int64_t dst_cap, void* stream);
+
 /* LZ4Codec.Wrap / Unwrap packet (src/LZ4/LZ4Codec.cs:510-543,574-599): u32le rawLen, u32le storedLen, payload. */
 int lz4b200_wrap(lz4b200_ctx* ctx, const void* src, int32_t n, int high_compression, void* dst, int32_t dst_cap);
 int lz4b200_unwrap_size(const void* src, int32_t n);

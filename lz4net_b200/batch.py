@@ -50,3 +50,50 @@ def compact(ctx: Context, slots: torch.Tensor, slot_off, lens, packed, out_off):
     native.check(native.lib().lz4b200_compact(ctx.handle, _p(slots), _p(slot_off), _p(lens),
                                               _p(packed) if packed is not None else 0, _p(out_off), lens.numel(), _stream()),
                  "compact")
+
+
+# ---- LZ4Stream framing on device memory --------------------------------------------------------------------------
+def _check_bytes(ctx: Context, t, what: str) -> int:
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.uint8:
+        raise TypeError(f"{what} must be a torch.uint8 tensor")
+    if t.device.type != "cuda" or t.device.index != ctx.device:
+        raise ValueError(f"{what} must be on cuda:{ctx.device}, the context's device (got {t.device})")
+    if t.dim() != 1 or not t.is_contiguous():
+        raise ValueError(f"{what} must be a 1-D contiguous tensor")
+    return t.numel()
+
+
+def stream_encode(ctx: Context, raw: torch.Tensor, block_size: int = 1 << 20, high_compression: bool = False) -> torch.Tensor:
+    """The LZ4Stream bytes of `raw` (what Context.stream_encode returns for the same bytes), built in device memory on the
+    current torch stream.  Returns a tensor of exactly the stream's length."""
+    n = _check_bytes(ctx, raw, "raw")
+    l = native.lib()
+    cap = int(l.lz4b200_stream_bound(n, block_size))
+    if cap < 0:
+        raise ValueError(f"block_size must be >= 1 (got {block_size})")
+    out = torch.empty(cap, dtype=torch.uint8, device=raw.device)
+    w = int(l.lz4b200_stream_encode_device(ctx.handle, _p(raw), n, block_size, int(high_compression), _p(out), cap,
+                                           torch.cuda.current_stream(raw.device).cuda_stream))
+    if w < 0:
+        raise native.Lz4B200Error(f"stream_encode failed ({w}): {native.last_error()}")
+    return out[:w]
+
+
+def stream_decode(ctx: Context, wire: torch.Tensor) -> torch.Tensor:
+    """Decode an LZ4Stream held in device memory, on the current torch stream.  Errors as Context.stream_decode:
+    a malformed chunk header raises EOFError, a chunk that does not decode ValueError."""
+    n = _check_bytes(ctx, wire, "wire")
+    l = native.lib()
+    st = torch.cuda.current_stream(wire.device).cuda_stream
+    total = int(l.lz4b200_stream_decoded_size_device(ctx.handle, _p(wire), n, st))
+    if total == native.E_FORMAT:
+        raise EOFError("LZ4Stream: unexpected end of stream / corrupt chunk header")     # EndOfStreamException
+    if total < 0:
+        raise native.Lz4B200Error(f"stream_decoded_size failed ({total}): {native.last_error()}")
+    out = torch.empty(total, dtype=torch.uint8, device=wire.device)
+    r = int(l.lz4b200_stream_decode_device(ctx.handle, _p(wire), n, _p(out), total, st))
+    if r == native.E_FORMAT:
+        raise ValueError("LZ4 block has been corrupted")
+    if r < 0:
+        raise native.Lz4B200Error(f"stream_decode failed ({r}): {native.last_error()}")
+    return out

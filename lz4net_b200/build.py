@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "liblz4b200.so")
-SOURCES = ["capi.cu", "decode.cu", "encode.cu", "util.cu", "framing.cpp"]
+SOURCES = ["capi.cu", "decode.cu", "encode.cu", "util.cu", "stream.cu", "framing.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -110,6 +110,8 @@ struct lz4b200_ctx {
     uint32_t* counters = nullptr;
     int next_counter = 0;
     DevBuf hc_arena, compact_tmp;
+    DevBuf stream_work, stream_table, stream_res;   // device framing: encoder slots + per-chunk metadata, chunk tables, walk result
+    PinBuf stream_host;                    // their results, read back by the host
     cudaEvent_t hc_done = nullptr;         // the HC state arena is shared: HC launches are chained through this event
     cudaEvent_t compact_done = nullptr;    // likewise the scan scratch of lz4b200_compact
     int decode_lanes = 16;                 // lanes per block for device-memory batches (+100 = output-staged variant)
@@ -424,6 +426,102 @@ int batch(lz4b200_ctx* c, const void* src, const int64_t* src_off, const int32_t
     return run_host(c, (const uint8_t*)src, src_off, src_len, (uint8_t*)dst, dst_off, dst_cap, out_len, n, op);
 }
 
+// ---- LZ4Stream framing on device memory (stream.cu) -------------------------------------------------------------------
+// The same byte stream as framing.cpp, without the bytes leaving the GPU.  Every call runs on the caller's stream and
+// waits for its own result there, so it is ordered after whatever the caller queued before it.
+
+// groups of chunks bound the device scratch, like the host framing: 256 MiB of raw bytes, and at most 4 Mi chunks
+// (44 bytes of metadata each) for tiny block sizes
+constexpr int64_t STREAM_GROUP_BYTES = 256 << 20, STREAM_GROUP_CHUNKS = 1 << 22;
+
+int64_t stream_encode_device(lz4b200_ctx* c, const uint8_t* src, int64_t n, int32_t bs, int hc, uint8_t* dst, cudaStream_t st)
+{
+    const int64_t chunks = (n + bs - 1) / bs;
+    const int64_t group = std::min(std::max<int64_t>(1, STREAM_GROUP_BYTES / bs), STREAM_GROUP_CHUNKS);
+    const int64_t gm = std::min(chunks, group);
+    // work buffer: slots (capacity == raw length, LZ4Stream.cs:243-246) | int64 off[m] | int64 pos[2m+1] | int32 len[m] | out[m] | sizes[2m]
+    const size_t slot_bytes = ((size_t)std::min<int64_t>(n, gm * bs) + 15) & ~(size_t)15;
+    CU(c->stream_work.reserve(slot_bytes + (size_t)gm * 44 + 64));
+    CU(c->stream_res.reserve(sizeof(StreamWalk)));
+    CU(c->stream_host.reserve(sizeof(StreamWalk)));
+    if (compact_tmp_bytes((int32_t)(2 * gm)) > c->compact_tmp.cap) { CU(cudaDeviceSynchronize()); CU(c->compact_tmp.reserve(compact_tmp_bytes((int32_t)(2 * gm)))); }
+    uint8_t* slots = (uint8_t*)c->stream_work.p;
+    int64_t* off = (int64_t*)(slots + slot_bytes);
+    int64_t* pos = off + gm;
+    int32_t* len = (int32_t*)(pos + 2 * gm + 1);
+    int32_t* out = len + gm;
+    int32_t* sizes = out + gm;
+    int64_t* h_total = (int64_t*)c->stream_host.p;
+    int64_t w = 0;
+    for (int64_t c0 = 0; c0 < chunks; c0 += group) {
+        const int32_t m = (int32_t)std::min(chunks - c0, group);
+        const int64_t base = c0 * bs;
+        cudaError_t e = launch_stream_layout(off, len, m, bs, n - base, st, &c->launches);
+        if (e != cudaSuccess) return cuda_fail(e, "stream layout launch");
+        BatchArgs a{src + base, off, len, slots, off, len, out, m};
+        int rc = run_device(c, a, hc ? 1 : 0, st); if (rc) return rc;
+        e = launch_stream_frame_sizes(len, out, m, hc, sizes, st, &c->launches);
+        if (e != cudaSuccess) return cuda_fail(e, "stream frame sizes launch");
+        CU(cudaStreamWaitEvent(st, c->compact_done, 0));            // the scan scratch is shared with lz4b200_compact
+        e = launch_compact(nullptr, nullptr, sizes, nullptr, pos, 2 * m, c->compact_tmp.p, c->compact_tmp.cap, c->dev, st, &c->launches);
+        if (e != cudaSuccess) return cuda_fail(e, "stream scan launch");
+        CU(cudaEventRecord(c->compact_done, st));
+        e = launch_stream_frame_write(src + base, off, len, slots, out, pos, m, hc, dst + w, st, &c->launches);
+        if (e != cudaSuccess) return cuda_fail(e, "stream frame write launch");
+        CU(cudaMemcpyAsync(h_total, pos + 2 * m, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));                              // the next group reuses the slots and needs w
+        w += *h_total;
+    }
+    return w;
+}
+
+// one walk of the chunk headers into the context's table (cap entries per table; 0 = count only); result on the host
+int stream_walk(lz4b200_ctx* c, const uint8_t* src, int64_t n, int64_t cap, cudaStream_t st, StreamWalk* out)
+{
+    CU(c->stream_res.reserve(sizeof(StreamWalk)));
+    CU(c->stream_host.reserve(sizeof(StreamWalk)));
+    if (cap) CU(c->stream_table.reserve(stream_table_bytes(cap)));
+    const StreamTable t = stream_table_at(c->stream_table.p, cap);
+    cudaError_t e = launch_stream_walk(src, n, cap, t, (StreamWalk*)c->stream_res.p, st, &c->launches);
+    if (e != cudaSuccess) return cuda_fail(e, "stream walk launch");
+    CU(cudaMemcpyAsync(c->stream_host.p, c->stream_res.p, sizeof(StreamWalk), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    *out = *(const StreamWalk*)c->stream_host.p;
+    return LZ4B200_OK;
+}
+
+int64_t stream_decode_device(lz4b200_ctx* c, const uint8_t* src, int64_t n, uint8_t* dst, int64_t dst_cap, cudaStream_t st)
+{
+    // every chunk has at least two header bytes; start from a guess for chunks of a few KiB and walk again if it was short
+    int64_t cap = std::max<int64_t>((int64_t)(c->stream_table.cap / stream_table_bytes(1)), std::min(n / 2 + 1, n / 4096 + 1024));
+    StreamWalk r;
+    int rc = stream_walk(c, src, n, cap, st, &r); if (rc) return rc;
+    if (r.status == 0 && std::max(r.n_stored, r.n_comp) > cap) {
+        cap = std::max(r.n_stored, r.n_comp);
+        rc = stream_walk(c, src, n, cap, st, &r); if (rc) return rc;
+    }
+    if (r.status < 0) return r.status;
+    if (r.total > dst_cap || (r.total > 0 && !dst)) return fail(LZ4B200_E_ARG, "destination too small");
+    if (std::max(r.n_stored, r.n_comp) > INT32_MAX) return fail(LZ4B200_E_ARG, "more than 2^31 chunks");
+    const StreamTable t = stream_table_at(c->stream_table.p, cap);
+    cudaError_t e = launch_scatter(src, t.st_src, t.st_len, dst, t.st_dst, (int32_t)r.n_stored, st, &c->launches);   // stored chunks (:295-299)
+    if (e != cudaSuccess) return cuda_fail(e, "stream stored-chunk copy launch");
+    if (r.n_comp > 0) {
+        const int32_t m = (int32_t)r.n_comp;
+        BatchArgs a{src, t.cp_src, t.cp_len, dst, t.cp_dst, t.cp_raw, t.cp_out, m};
+        rc = run_device(c, a, 2, st); if (rc) return rc;
+        // LZ4Codec.Decode(..., knownOutputLength: true) throws unless exactly compLen bytes were consumed
+        // (src/LZ4ps/LZ4Codec.Safe.cs:539-542)
+        StreamWalk* res = (StreamWalk*)c->stream_res.p;
+        e = launch_stream_verdict(t.cp_out, t.cp_len, m, &res->bad, c->dev, st, &c->launches);
+        if (e != cudaSuccess) return cuda_fail(e, "stream verdict launch");
+        CU(cudaMemcpyAsync(c->stream_host.p, res, sizeof(StreamWalk), cudaMemcpyDeviceToHost, st));
+    }
+    CU(cudaStreamSynchronize(st));
+    if (r.n_comp > 0 && ((const StreamWalk*)c->stream_host.p)->bad) return LZ4B200_E_FORMAT;
+    return r.total;
+}
+
 // The single-block entry points are re-entrant like the reference's (SURVEY 8b "Threading"): every calling thread gets
 // a context of its own (streams + staging buffers), created on first use and destroyed with the thread.
 struct ThreadCtx {
@@ -517,6 +615,7 @@ void lz4b200_destroy(lz4b200_ctx* c)
         if (s.stream) cudaStreamDestroy(s.stream);
     }
     c->hc_arena.release(); c->compact_tmp.release();
+    c->stream_work.release(); c->stream_table.release(); c->stream_res.release(); c->stream_host.release();
     if (c->hc_done) cudaEventDestroy(c->hc_done);
     if (c->compact_done) cudaEventDestroy(c->compact_done);
     if (c->counters) cudaFree(c->counters);
@@ -677,6 +776,41 @@ int lz4b200_peer_copy(void* dst, const void* src, int64_t bytes, void* stream)
     CU(cudaSetDevice(cur));
     CU(cudaMemcpyPeerAsync(dst, dev[0], src, dev[1], (size_t)bytes, (cudaStream_t)stream));   // a copy-engine transfer
     return LZ4B200_OK;
+}
+
+int64_t lz4b200_stream_encode_device(lz4b200_ctx* c, const void* src, int64_t n, int32_t block_size, int high_compression,
+                                     void* dst, int64_t dst_cap, void* stream)
+{
+    if (!c || n < 0 || block_size < 1 || (n > 0 && (!src || !dst))) return fail(LZ4B200_E_ARG, "bad argument");
+    if (dst_cap < lz4b200_stream_bound(n, block_size)) return fail(LZ4B200_E_ARG, "dst_cap is below lz4b200_stream_bound");
+    if (n == 0) return 0;
+    std::lock_guard<std::mutex> lock(c->mu);
+    DeviceGuard g(c->device);
+    if (!g.ok) return fail(LZ4B200_E_CUDA, "cudaSetDevice failed");
+    return stream_encode_device(c, (const uint8_t*)src, n, block_size, high_compression ? 1 : 0, (uint8_t*)dst, (cudaStream_t)stream);
+}
+
+int64_t lz4b200_stream_decoded_size_device(lz4b200_ctx* c, const void* src, int64_t n, void* stream)
+{
+    if (!c || n < 0 || (n > 0 && !src)) return fail(LZ4B200_E_ARG, "bad argument");
+    if (n == 0) return 0;
+    std::lock_guard<std::mutex> lock(c->mu);
+    DeviceGuard g(c->device);
+    if (!g.ok) return fail(LZ4B200_E_CUDA, "cudaSetDevice failed");
+    StreamWalk r;
+    const int rc = stream_walk(c, (const uint8_t*)src, n, 0, (cudaStream_t)stream, &r);
+    if (rc) return rc;
+    return r.status < 0 ? r.status : r.total;
+}
+
+int64_t lz4b200_stream_decode_device(lz4b200_ctx* c, const void* src, int64_t n, void* dst, int64_t dst_cap, void* stream)
+{
+    if (!c || n < 0 || (n > 0 && !src)) return fail(LZ4B200_E_ARG, "bad argument");
+    if (n == 0) return dst_cap < 0 ? fail(LZ4B200_E_ARG, "destination too small") : 0;
+    std::lock_guard<std::mutex> lock(c->mu);
+    DeviceGuard g(c->device);
+    if (!g.ok) return fail(LZ4B200_E_CUDA, "cudaSetDevice failed");
+    return stream_decode_device(c, (const uint8_t*)src, n, (uint8_t*)dst, dst_cap, (cudaStream_t)stream);
 }
 
 int lz4b200_compress_limitedOutput(const char* s, char* d, int isize, int cap) { return single(s, d, isize, cap, 0); }

@@ -4,8 +4,10 @@
 // LZ4Codec.Encode/EncodeHC with capacity == block length, and writes  varint(flags) varint(rawLen) [varint(compLen)]
 // payload  per chunk (FlushCurrentChunk :239-269; reader AcquireNextChunk :274-312; varints :167-187,225-236).
 // Here the same byte stream is produced / consumed with ONE batched GPU call for all chunks of a buffer.
-// Pure host code: no kernels, no codec arithmetic -- that all lives behind lz4b200_{encode,decode}_batch.
+// Pure host code: no kernels, no codec arithmetic -- that all lives behind lz4b200_{encode,decode}_batch.  The chunk
+// header codec is lz4_stream.cuh, which the device framing of stream.cu / capi.cu uses as well.
 #include "../../include/lz4b200.h"
+#include "lz4_stream.cuh"
 
 #include <algorithm>
 #include <cstdint>
@@ -14,56 +16,19 @@
 
 namespace {
 
-enum : uint64_t { FLAG_COMPRESSED = 1, FLAG_HC = 2 };          // ChunkFlags, LZ4Stream.cs:43-58
-
-inline int varint_size(uint64_t v) { int n = 1; while (v >>= 7) n++; return n; }
-
-inline uint8_t* put_varint(uint8_t* p, uint64_t v)             // LZ4Stream.cs:225-236
-{
-    for (;;) {
-        uint8_t b = (uint8_t)(v & 0x7F);
-        v >>= 7;
-        *p++ = (uint8_t)(b | (v ? 0x80 : 0));
-        if (!v) return p;
-    }
-}
-
-// LZ4Stream.cs:167-187.  Returns 1 = value read, 0 = clean end of data before the first byte, -1 = truncated.
-inline int get_varint(const uint8_t* s, int64_t n, int64_t* pos, uint64_t* out)
-{
-    uint64_t r = 0; int count = 0;
-    for (;;) {
-        if (*pos >= n) return count == 0 ? 0 : -1;
-        uint8_t b = s[(*pos)++];
-        r += (uint64_t)(b & 0x7F) << count;
-        count += 7;
-        if (!(b & 0x80) || count >= 64) break;
-    }
-    *out = r;
-    return 1;
-}
-
-struct Chunk { int64_t payload; int32_t raw; int32_t stored; bool compressed; };
+using namespace lz4b200::lz4s;
 
 // walk the chunk headers of a whole stream; returns total raw size or a negative status
 int64_t walk(const uint8_t* s, int64_t n, std::vector<Chunk>* out)
 {
     int64_t pos = 0, total = 0;
     for (;;) {
-        uint64_t flags, raw, clen;
-        int r = get_varint(s, n, &pos, &flags);
-        if (r == 0) return total;                               // legitimate end (LZ4Stream.cs:281)
-        if (r < 0) return LZ4B200_E_FORMAT;
-        if (get_varint(s, n, &pos, &raw) != 1) return LZ4B200_E_FORMAT;
-        const bool comp = (flags & FLAG_COMPRESSED) != 0;
-        clen = raw;
-        if (comp && get_varint(s, n, &pos, &clen) != 1) return LZ4B200_E_FORMAT;
-        const int32_t rawi = (int32_t)raw, cleni = (int32_t)clen;             // the reference casts to int (:286-287)
-        if (rawi < 0 || cleni < 0 || cleni > rawi) return LZ4B200_E_FORMAT;   // :288 corrupted
-        if (pos + cleni > n) return LZ4B200_E_FORMAT;                         // :293 short read
-        if (comp && (flags >> 2) != 0) return LZ4B200_E_FORMAT;               // :301-303 multi-pass chunks unsupported
-        if (out) out->push_back(Chunk{pos, rawi, cleni, comp});
-        pos += cleni; total += rawi;
+        Chunk c;
+        const int r = walk_step(s, n, &pos, &c);
+        if (r == 0) return total;
+        if (r < 0) return r;
+        if (out) out->push_back(c);
+        total += c.raw;
     }
 }
 
@@ -104,9 +69,9 @@ int64_t lz4b200_stream_encode(lz4b200_ctx* ctx, const void* src, int64_t n, int3
         if (rc != LZ4B200_OK) return rc;
         for (int64_t i = 0; i < m; i++) {
             const int32_t raw = sl[i], clen = out[i];
-            const bool comp = clen > 0 && clen < raw;                         // LZ4Stream.cs:248-255
+            const bool comp = chunk_compressed(raw, clen);                   // LZ4Stream.cs:248-255
             uint8_t* p = d + w;
-            p = put_varint(p, (comp ? FLAG_COMPRESSED : 0) | (hc ? FLAG_HC : 0));
+            p = put_varint(p, chunk_flags(comp, hc != 0));
             p = put_varint(p, (uint64_t)raw);
             if (comp) p = put_varint(p, (uint64_t)clen);
             std::memcpy(p, comp ? slots.data() + dof[i] : s + so[i], (size_t)(comp ? clen : raw));

@@ -123,6 +123,15 @@ cudaError_t launch_compact(const uint8_t* slots, const int64_t* slot_off, const 
     return cudaGetLastError();
 }
 
+cudaError_t launch_scatter(const uint8_t* src, const int64_t* src_off, const int32_t* len, uint8_t* dst, const int64_t* dst_off,
+                           int32_t n, cudaStream_t stream, int64_t* launches)
+{
+    if (n <= 0) return cudaSuccess;
+    gather_blocks<<<(n + 7) / 8, 256, 0, stream>>>(src, src_off, len, dst, dst_off, n);
+    if (launches) ++*launches;
+    return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // Synthetic entropy classes -- the CUDA twin of lz4net_b200/synth.py (same formulas, same bytes).
 // ---------------------------------------------------------------------------------------------------------------------

@@ -37,6 +37,9 @@ SIGNATURES = {
     "lz4b200_stream_encode": (_L, [_P, _P, _L, C.c_int32, _I, _P, _L]),
     "lz4b200_stream_decoded_size": (_L, [_P, _L]),
     "lz4b200_stream_decode": (_L, [_P, _P, _L, _P, _L]),
+    "lz4b200_stream_encode_device": (_L, [_P, _P, _L, C.c_int32, _I, _P, _L, _P]),
+    "lz4b200_stream_decoded_size_device": (_L, [_P, _P, _L, _P]),
+    "lz4b200_stream_decode_device": (_L, [_P, _P, _L, _P, _L, _P]),
     "lz4b200_wrap": (_I, [_P, _P, C.c_int32, _I, _P, C.c_int32]),
     "lz4b200_unwrap_size": (_I, [_P, C.c_int32]),
     "lz4b200_unwrap": (_I, [_P, _P, C.c_int32, _P, C.c_int32]),
